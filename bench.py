@@ -14,6 +14,10 @@ re-linearisation).  `python bench.py --gpus N --steps K --warmup W` (under torch
   * `cpu_baseline` (N = 1, rank 0): the CPU oracle (port of the Theia+Ceres path; Ceres itself is not
     installable here) on a bounded sample.
 `--impl reference` times that CPU restatement alone with all host threads.
+`--dump-outputs DIR` (one process) writes what the timed solve computed as float64 arrays DIR/<name>.npy: the cameras,
+the intrinsics, a fixed seeded sample of the points and the per-iteration costs.  When the solve reaches the fp64 floor
+before K iterations, these are its results there, not those of the restarts that fill up K (which repeat its start).  The
+scene is seeded, so the same arguments give the same inputs and two builds can be compared output for output.
 """
 import argparse
 import json
@@ -469,9 +473,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-experiments", action="store_true", help="skip the diagnostic pass over the compiled-in experiment switches")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed solve computed as DIR/<name>.npy (float64, "
+                                                          "about 9 MB for c3_10kcam); bundle adjustment on one GPU")
     ap.add_argument("--experiments-child", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--device", type=int, default=0, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "c5_matcher" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes the bundle-adjustment result of one GPU (no --impl reference, c5_matcher or WORLD_SIZE > 1)")
     if args.experiments_child:
         return experiments_child(args.workload, args.steps, args.device)
     if args.workload == "c5_matcher":
@@ -574,8 +584,8 @@ def main():
     barrier()
     tw0 = time.time()
     t0 = time.perf_counter()
-    iters, dev_s, launches_local, pcg_total, solves, s = 0, 0.0, 0.0, 0, 0, None
-    while iters < K and solves < 8:
+    iters, dev_s, launches_local, pcg_total, solves, s, result = 0, 0.0, 0.0, 0, 0, None, None
+    while iters < K:
         if solves > 0:
             eng.reset_parameters(init)
         eng.set_max_iterations(K - iters)
@@ -589,20 +599,25 @@ def main():
         launches_local += float(si.num_kernel_launches)
         pcg_total += int(si.num_linear_solver_iterations)
         if got <= 0:
-            break
+            raise RuntimeError("a solve from the initial estimate ran no LM iteration (%d of %d done): %s" % (iters, K, si.message))
+        if args.dump_outputs and solves == 1 and iters < K:
+            result = init.copy()  # the restarts overwrite the first solve's result on the device (the copy is not device-timed)
+            eng.download(result)
     barrier()
     wall = time.perf_counter() - t0
     clocks = sampler.stop(tw0, time.time())
     prof = eng.profile()
     stages = eng.profile_stages()
     eng.set_profiling(False)
+    if args.dump_outputs:
+        if result is None:
+            result = init.copy()
+            eng.download(result)
+        write_outputs(args.dump_outputs, result, s.costs)
     t_max = max_over_ranks(dev_s if dev_s > 0 else wall)  # device time of the iterations; the wall clock only if the engine reported none
     launches = sum_over_ranks(launches_local)
     note = None if solves == 1 else ("%d LM iterations timed as %d solves restarted from the initial estimate (the first stopped after %d: %s)"
                                      % (iters, solves, s.num_iterations - 1, s.message))
-    if iters != K:
-        note = "only %d of %d LM iterations ran: %s" % (iters, K, s.message)
-    iters = max(iters, 1)
     value = n_obs_total * iters / t_max
     # ---- roofline of the dominant kernel (implicit-Schur matvec; DESIGN.md section 5)
     peak, peak_src = load_peaks()
@@ -672,6 +687,20 @@ def main():
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_POINTS = 1 << 18  # points written by --dump-outputs: a seeded sample of this many rows when the scene has more (8 MB)
+
+
+def write_outputs(out_dir, p, costs):
+    """--dump-outputs: the adjusted parameters a caller of the timed path downloads (cameras [n_cam, 6], intrinsics [n_group, 10],
+    points [n_pt, 4], sampled to DUMP_POINTS sorted rows by a fixed seed) and the per-iteration costs of the solve."""
+    os.makedirs(out_dir, exist_ok=True)
+    pt = p.pt
+    if len(pt) > DUMP_POINTS:
+        pt = pt[np.sort(np.random.default_rng(0).choice(len(pt), DUMP_POINTS, replace=False))]
+    for name, a in (("cameras", p.ext), ("intrinsics", p.intr), ("points", pt), ("costs", costs)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float64))
 
 
 def full_cam_bytes(p):

@@ -1,9 +1,13 @@
 """Generates tests/golden/fountain11_ir.npz from the reference's own fixtures
-  /root/reference/data/sfm/fountain11.bin      (a reconstruction saved by Theia after ITS OWN bundle adjustment)
-  /root/reference/data/sfm/gt_fountain11.bin   (ground-truth cameras of Strecha fountain-P11)
+  data/sfm/fountain11.bin      (a reconstruction saved by Theia after ITS OWN bundle adjustment)
+  data/sfm/gt_fountain11.bin   (ground-truth cameras of Strecha fountain-P11)
 used by incremental_reconstruction_estimator_test.cc:52-160.  The reference cannot run here (C++ needing Ceres), but its
 saved OUTPUT travels: the flattened IR of that reconstruction pins our cost function against a state the reference's
-BA produced (tests/test_fountain_fixture.py).    Run:  python tests/golden/make_fountain_fixture.py
+BA produced (tests/test_fountain_fixture.py).    Run:  python tests/golden/make_fountain_fixture.py <TheiaSfM>/data/sfm
+
+The file is stored compacted, losslessly, to stay small: pixel coordinates as float32 (every one of them is exactly
+representable, asserted below), pt and obs_xy as the byte planes of their column-major data (the sign / exponent bytes
+then compress well), obs_pt as differences of consecutive entries.  tests/helpers.py:fountain_problem() undoes it.
 """
 import os
 import sys
@@ -14,12 +18,16 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 import theia_cereal  # noqa: E402
 
-DATA = "/root/reference/data/sfm"
+
+def byte_planes(a):
+    """[n, k] -> uint8 [itemsize, n * k]: byte j of every element of the column-major data in row j."""
+    a = np.ascontiguousarray(np.asarray(a).T)
+    return np.ascontiguousarray(a.view(np.uint8).reshape(-1, a.dtype.itemsize).T)
 
 
-def main():
-    rec = theia_cereal.reconstruction(open(os.path.join(DATA, "fountain11.bin"), "rb").read())
-    gt = theia_cereal.reconstruction(open(os.path.join(DATA, "gt_fountain11.bin"), "rb").read())
+def main(data):
+    rec = theia_cereal.reconstruction(open(os.path.join(data, "fountain11.bin"), "rb").read())
+    gt = theia_cereal.reconstruction(open(os.path.join(data, "gt_fountain11.bin"), "rb").read())
     assert rec["consumed"] == rec["total"] and gt["consumed"] == gt["total"]
     vids = sorted(rec["views"])
     tids = sorted(t for t in rec["tracks"] if rec["tracks"][t]["est"])
@@ -41,10 +49,13 @@ def main():
     gt_ext = np.array([gt_by_name[n]["ext"] for n in names])
     gt_intr = np.array([gt_by_name[n]["intr"] for n in names])
     out = os.path.join(HERE, "fountain11_ir.npz")
-    np.savez_compressed(out, names=np.array(names), ext=ext, intr=intr, pt=pt, obs_cam=np.array(oc, np.int32),
-                        obs_pt=np.array(op, np.int32), obs_xy=np.array(oxy), gt_ext=gt_ext, gt_intr=gt_intr)
+    oxy = np.array(oxy)
+    assert np.array_equal(oxy.astype(np.float32), oxy) and len(vids) < 256 and len(tids) < 2 ** 15
+    np.savez_compressed(out, names=np.array(names), ext=ext, intr=intr, pt=byte_planes(pt), obs_cam=np.array(oc, np.uint8),
+                        obs_pt=np.diff(np.array(op), prepend=0).astype(np.int16), obs_xy=byte_planes(oxy.astype(np.float32)),
+                        gt_ext=gt_ext, gt_intr=gt_intr)
     print("wrote", out, "cams", len(vids), "points", len(tids), "obs", len(oc), "bytes", os.path.getsize(out))
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

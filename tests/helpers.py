@@ -57,7 +57,12 @@ FOUNTAIN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "f
 def fountain_problem(intrinsics_to_optimize=_abi.INTR_NONE):
     """The reference's fountain-11 reconstruction as a Problem (shared PINHOLE intrinsics; constant by default, as in
     the run that produced it: the stored intrinsics equal the ground-truth calibration exactly)."""
-    g = np.load(FOUNTAIN)
+    g = dict(np.load(FOUNTAIN))
+    # undo the lossless compaction of tests/golden/make_fountain_fixture.py
+    for k, dtype, cols in (("pt", np.float64, 4), ("obs_xy", np.float32, 2)):
+        g[k] = np.ascontiguousarray(g[k].T).view(dtype).reshape(cols, -1).T.astype(np.float64)
+    g["obs_cam"] = g["obs_cam"].astype(np.int32)
+    g["obs_pt"] = np.cumsum(g["obs_pt"], dtype=np.int32)
     n = len(g["names"])
     mask = _abi.constant_intrinsics_mask(_abi.MODEL_PINHOLE, intrinsics_to_optimize)
     p = _abi.Problem(g["ext"], np.zeros(n, np.uint8), np.zeros(n, np.int32), [_abi.MODEL_PINHOLE], g["intr"], [mask], g["pt"],

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 PRELUDE = """
@@ -42,6 +44,51 @@ bench.main()
     assert line["steps"] == 2 and line["steps_requested"] == 2 and line["value"] > 0 and line["obs_passes_per_s"] >= line["value"]
 
 
+def _bench_line(*argv):
+    out = _run("""
+import bench
+bench.run_microbench = lambda d: None
+sys.argv = ["bench.py", "--workload", "c1_50cam", "--warmup", "1", "--no-cpu-baseline", "--no-e2e", "--no-experiments"] + %r
+bench.main()
+""" % list(argv))
+    assert out.returncode == 0, out.stderr[-2000:]
+    return json.loads(out.stdout.strip().splitlines()[-1])
+
+
+def test_bench_runs_exactly_the_requested_steps():
+    """Each solve of this scene stops at its fp64 floor after a few dozen LM iterations at most; the rest of the 400 come from
+    solves restarted at the initial estimate, as many as it takes."""
+    line = _bench_line("--steps", "400")
+    assert line["steps"] == line["steps_requested"] == 400 and line["solves_in_timed_region"] > 8
+
+
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs writes the timed solve's result; a second run with the same arguments starts from the same inputs."""
+    dumps = []
+    for run in ("a", "b"):
+        assert _bench_line("--steps", "3", "--dump-outputs", str(tmp_path / run))["steps"] == 3
+        dumps.append({f.stem: np.load(f) for f in (tmp_path / run).iterdir()})
+    a, b = dumps
+    assert {k: v.shape for k, v in a.items()} == {"cameras": (50, 6), "intrinsics": (1, 10), "points": (5000, 4), "costs": (4,)}
+    for k in a:
+        assert a[k].dtype == np.float64 and np.allclose(a[k], b[k], rtol=1e-12, atol=0), k
+    assert a["costs"][3] < a["costs"][0]
+
+
+def test_dump_outputs_of_the_largest_scene_stay_under_64_mb(tmp_path):
+    """c3_10kcam: 2 M points (64 MB of float64 alone) are written as a fixed, sorted sample."""
+    import bench
+
+    class P:
+        ext, intr, pt = np.zeros((10_000, 6)), np.zeros((1, 10)), np.arange(8.0 * 10 ** 6).reshape(-1, 4)
+    bench.write_outputs(str(tmp_path / "a"), P, np.ones(21))
+    bench.write_outputs(str(tmp_path / "b"), P, np.ones(21))
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 << 20
+    pts = np.load(tmp_path / "a" / "points.npy")
+    assert pts.shape == (bench.DUMP_POINTS, 4) and np.all(np.diff(pts[:, 0]) > 0) and np.all(pts[:, 0] % 4 == 0)
+    assert np.array_equal(pts, np.load(tmp_path / "b" / "points.npy"))
+
+
 def test_smoke_logic():
     out = _run("import __graft_entry__ as g\ng.smoke()\n")
     assert out.returncode == 0, out.stderr[-2000:]
@@ -72,9 +119,11 @@ bench.experiments_child("c1_50cam", 2, 0)
         assert set(d["stage_ms_per_step"]) >= {"matvec", "linearize", "precond_ext", "precond_intr", "rhs", "backsub", "candidate_cost"}
 
 
-def test_bench_experiments_parent_survives_a_failing_child():
+def test_bench_experiments_parent_survives_a_failing_child(monkeypatch):
     """Without a GPU the real child cannot create an engine: every variant reports its error (or the child dies), the parent
-    returns a dictionary either way and never raises."""
+    returns a dictionary either way and never raises.  The child inherits an empty CUDA_VISIBLE_DEVICES, so it sees no GPU on
+    a machine that has one too."""
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     sys.path.insert(0, ROOT)
     import bench
     res = bench.run_experiments("c1_50cam", 1, 0, timeout=240)
@@ -82,7 +131,7 @@ def test_bench_experiments_parent_survives_a_failing_child():
     assert all(("error" in v or v.get("rc") != 0) for k, v in res.items() if k != "note") or "note" in res
 
 
-def test_bench_main_and_experiments_child_against_the_emulated_engine():
+def test_bench_main_and_experiments_child_against_the_emulated_engine(tmp_path):
     """The same two entry points through the REAL ctypes binding and the real engine code (tests/emu SIMT-emulation build) instead of the
     mock: catches attribute / signature drift between engine.py and what bench.py expects (it did: minimize()'s summary had no rc)."""
     emu = os.path.join(ROOT, "tests", "emu")
@@ -100,14 +149,15 @@ os.environ["TBA_BENCH_MATCHER_N"] = "32"
 import bench
 bench.run_microbench = lambda d: None
 bench.run_experiments = lambda w, k, d: {"skipped": True}
-sys.argv = ["bench.py", "--workload", "c1_50cam", "--steps", "1", "--warmup", "1", "--no-cpu-baseline", "--no-e2e"]
+sys.argv = ["bench.py", "--workload", "c1_50cam", "--steps", "1", "--warmup", "1", "--no-cpu-baseline", "--no-e2e", "--dump-outputs", %r]
 bench.main()
 bench.experiments_child("c1_50cam", 1, 0)
-""" % (ROOT, emu, emu)
+""" % (ROOT, emu, emu, str(tmp_path))
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [json.loads(ln) for ln in out.stdout.strip().splitlines() if ln.startswith("{")]
     main, child = lines[0], lines[1:]
+    assert np.load(tmp_path / "points.npy").shape == (5000, 4) and np.load(tmp_path / "costs.npy").shape == (2,)
     assert main["steps"] == 1 and main["gpu_launches"] > 0 and set(main["stage_ms_per_step"]) == set(__import__("bench").VARIANTS and
                                                                                                       ("matvec", "linearize", "precond_ext", "precond_intr", "rhs", "backsub", "candidate_cost", "prepare_fused"))
     assert [d["variant"] for d in child] == [v[0] for v in __import__("bench").VARIANTS] + ["matcher_sample"]
