@@ -87,6 +87,34 @@ using namespace tba;
 
 static_assert(TILE == kPackTile && MAXP == kPackMaxPoints, "tba_pack.h and tba_kernels.cuh disagree on the tile shape");
 
+// A persistent kernel (one CTA per SM at most) with its launch shape.
+template <class Fn>
+struct PersistentKernel {
+  Fn fn = nullptr;
+  int nw = 0;       // warps per CTA
+  size_t smem = 0;  // dynamic shared memory
+};
+
+// The kernel instantiations an uploaded problem runs, chosen once by tba_upload (select_kernels) from the intrinsics column set,
+// the camera models and the switches read by tba_create.  The stages launch through it.
+struct KernelSet {
+  void (*linearize)(DevProblem, double*, double*, double*) = nullptr;
+  // the implicit Schur operator by MODE (0 matvec, 1 reduced rhs, 2 back-substitution): tile per CTA, and streaming over the normal tiles
+  void (*schur[3])(DevProblem, const double*, double*, double*, const int*, int) = {};
+  size_t schur_smem = 0;
+  PersistentKernel<void (*)(DevProblem, const double*, double*, double*, const int*, int, P2pDev)> schur_stream[3];
+  PersistentKernel<void (*)(DevProblem, double*, double*, double*, double*, int)> prepare_stream;
+  void (*precond_ext)(DevProblem, double*, int) = nullptr;
+  void (*precond_intr)(DevProblem, double*, int) = nullptr;
+  size_t precond_intr_smem = 0;
+  void (*cost)(DevProblem, const double*, const double*, const double*, const double*, double*) = nullptr;
+  void (*adjust_tracks)(DevProblem, const long long*, const int*, PointLmOptions, uint8_t*, double*) = nullptr;
+  void (*filter_tracks)(DevProblem, const long long*, const int*, double, double, uint8_t*, double*) = nullptr;
+  void (*estimate_tracks)(DevProblem, const long long*, const int*, const double*, TrackEstimatorOptions, uint8_t*, double*) = nullptr;
+  void (*block_pass[2][2])(DevProblem, BlockPassArgs) = {};  // [KIND][COST_ONLY]
+  int n_stream_tiles = 0;  // leading tiles the streaming kernels take: the normal tiles, or 0 when they are switched off
+};
+
 struct tba_context {
   int device = 0, rank = 0, world = 1;
   cudaStream_t stream = nullptr;
@@ -94,8 +122,8 @@ struct tba_context {
   std::string err;
   bool uploaded = false;
   tba_options opt;
-  uint32_t imask = 0;  // instantiated intrinsics column set
-  int NI = 0, NJ = 14;
+  int NI = 0, NJ = 14;  // stored intrinsics columns, Jacobian doubles per observation
+  KernelSet ks;
   DevProblem P;
   int n_cam = 0, n_group = 0, n_pt = 0, n_tiles = 0;
   int64_t n_obs = 0, n_slots = 0;
@@ -152,7 +180,6 @@ struct tba_context {
   double trace_pcg_gpu_ms = 0.0;  // TBA_TRACE_LM: device-side span of the PCG launches (first launch .. state copy), summed over a minimize
   bool pcg_fused = true;    // one vector kernel per CG iteration (k_pcg_fused, grid barriers between its phases); TBA_PCG=split: k_pcg_c / k_pcg_a / k_pcg_b
   bool stream_schur = true; // persistent streaming k_schur_stream over the normal tiles; TBA_MATVEC=tile: the tile-per-CTA k_schur everywhere
-  int n_normal_tiles = 0;   // tiles whose tracks fit a warp slice (they precede the long tiles)
   // fused matvec + all-reduce over peer memory (P2pDev, tba_kernels.cuh): world > 1, every peer reachable, TBA_P2P != 0
   bool p2p_enabled = true, p2p_ok = false, p2p_use = false;
   size_t p2p_cap = 0;
@@ -244,24 +271,18 @@ void prof_end(tba_context* c, int which, int begin) {
   c->ev_spans[which].push_back({begin, (int)c->ev_pool.size() - 1});
 }
 
+// The intrinsics column set the kernels are compiled for: the first of these that covers every free intrinsics column.
 const uint32_t kMasks[] = {0x000u, 0x001u, 0x061u, 0x0E1u, 0x07Fu, 0x3FFu};
-
-#define DISPATCH_IMASK(mask, F) \
-  switch (mask) {               \
-    case 0x000u: F(0x000u); break; \
-    case 0x001u: F(0x001u); break; \
-    case 0x061u: F(0x061u); break; \
-    case 0x0E1u: F(0x0E1u); break; \
-    case 0x07Fu: F(0x07Fu); break; \
-    default: F(0x3FFu); break;  \
-  }
+uint32_t intrinsics_mask(uint32_t union_free) {
+  for (uint32_t m : kMasks) if ((union_free & ~m) == 0) return m;
+  return 0x3FFu;
+}
 
 int allreduce_sum(tba_context* c, double* buf, size_t n) {
   if (c->world == 1) return TBA_OK;
   NCCL_OK(c, g_nccl.AllReduce(buf, buf, n, ncclDouble, ncclSum, c->comm, c->stream));
   return TBA_OK;
 }
-size_t schur_smem(const tba_context* c) { return (size_t)(c->NJ + 2) * TILE * sizeof(double); }
 
 double* lin_g(tba_context* c) { return c->lin.p; }
 double* lin_cn(tba_context* c) { return c->lin.p + c->P.ncs; }
@@ -269,6 +290,8 @@ double* lin_scal(tba_context* c) { return c->lin.p + 2 * (size_t)c->P.ncs; }
 // grid of the per-point / per-element streaming kernels (256 threads per CTA): enough CTAs to cover the latency of a dependent
 // load chain (8 per SM), not more than the work
 int small_grid(const tba_context* c, int64_t n_items) { return (int)std::max<int64_t>(1, std::min<int64_t>((n_items + 255) / 256, (int64_t)c->n_sm * 8)); }
+// grid of the persistent streaming kernels: one CTA per SM at most, not more than the slices of 32 observations need
+int persistent_grid(const tba_context* c, int nw, int n_slices) { return std::max(1, std::min(c->n_sm, (n_slices + nw - 1) / nw)); }
 
 // scal layout: 0 cost, 1 fixed cost, 2 failed evals, 3 model cost change, 4 |delta_cs|^2, 5 |delta_pt|^2,
 //              6 |x_cs|^2, 7 |x_pt|^2
@@ -276,6 +299,21 @@ int read_scal(tba_context* c, const double* dev, int n, double* out) {
   CUDA_OK(c, cudaMemcpyAsync(c->h_scal, dev, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
   CUDA_OK(c, cudaStreamSynchronize(c->stream));
   memcpy(out, c->h_scal, n * sizeof(double));
+  return TBA_OK;
+}
+// Sums n doubles on the device over the ranks, then reads them to the host.
+int allreduce_read(tba_context* c, double* dev, int n, double* out) {
+  const int rc = allreduce_sum(c, dev, (size_t)n);
+  return rc ? rc : read_scal(c, dev, n, out);
+}
+// Sums n host values over the ranks in place (through scal2): every rank gets the same values back.
+int allreduce_host(tba_context* c, double* v, size_t n) {
+  CUDA_OK(c, c->scal2.alloc(std::max<size_t>(n, 16)));
+  CUDA_OK(c, cudaMemcpyAsync(c->scal2.p, v, n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+  const int rc = allreduce_sum(c, c->scal2.p, n);
+  if (rc) return rc;
+  CUDA_OK(c, cudaMemcpyAsync(v, c->scal2.p, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_OK(c, cudaStreamSynchronize(c->stream));
   return TBA_OK;
 }
 
@@ -290,26 +328,7 @@ int stage_linearize(tba_context* c, double* cost, double* fixed, bool* ok, doubl
   LAUNCH(c, k_cam_prep, (P.n_cam + 127) / 128, 128, 0, P.n_cam, P.ext, P.cam_rec, P.cam_s4);
   if (P.n_tiles > 0) {
     const int pb = prof_begin(c);
-    if (c->has_ext_models) {  // FISHEYE / FOV / DIVISION_UNDISTORTION present: the dual-number instantiation, all 10 columns
-      auto kfn = k_linearize<0x3FFu, true>;
-      LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, lin_g(c), lin_cn(c), c->rep.p);
-    } else if (c->exp_lin_occ && c->exp_tred) {
-#define F(M) { auto kfn = k_linearize<M, false, true, 3>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, lin_g(c), lin_cn(c), c->rep.p); }
-      DISPATCH_IMASK(c->imask, F)
-#undef F
-    } else if (c->exp_lin_occ) {
-#define F(M) { auto kfn = k_linearize<M, false, false, 3>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, lin_g(c), lin_cn(c), c->rep.p); }
-      DISPATCH_IMASK(c->imask, F)
-#undef F
-    } else if (c->exp_tred) {
-#define F(M) { auto kfn = k_linearize<M, false, true>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, lin_g(c), lin_cn(c), c->rep.p); }
-      DISPATCH_IMASK(c->imask, F)
-#undef F
-    } else {
-#define F(M) LAUNCH(c, k_linearize<M>, P.n_tiles, TILE, 0, P, lin_g(c), lin_cn(c), c->rep.p)
-      DISPATCH_IMASK(c->imask, F)
-#undef F
-    }
+    LAUNCH(c, c->ks.linearize, P.n_tiles, TILE, 0, P, lin_g(c), lin_cn(c), c->rep.p);
     prof_end(c, 1, pb);
     LAUNCH(c, k_fold, 1, REPW, 0, c->rep.p, lin_g(c) + P.ne, lin_cn(c) + P.ne, lin_scal(c));
   }
@@ -407,17 +426,11 @@ int p2p_setup(tba_context* c, int ncs) {
       inbox[q] = (double*)pi; flags[q] = (unsigned long long*)pf;
     }
   }
-  // every rank must agree (a min-reduction of the success flags through the existing all-reduce)
-  {
-    CUDA_OK(c, c->scal2.alloc(16));
-    const double v = ok ? 0.0 : 1.0;
-    CUDA_OK(c, cudaMemcpyAsync(c->scal2.p, &v, 8, cudaMemcpyHostToDevice, c->stream));
-    NCCL_OK(c, g_nccl.AllReduce(c->scal2.p, c->scal2.p, 1, ncclDouble, ncclSum, c->comm, c->stream));
-    double failed = 0;
-    CUDA_OK(c, cudaMemcpyAsync(&failed, c->scal2.p, 8, cudaMemcpyDeviceToHost, c->stream));
-    CUDA_OK(c, cudaStreamSynchronize(c->stream));
-    if (failed != 0.0) { p2p_release(c); return TBA_OK; }
-  }
+  // every rank must agree: the number of ranks that failed, summed over the ranks
+  double failed = ok ? 0.0 : 1.0;
+  const int rc = allreduce_host(c, &failed, 1);
+  if (rc) return rc;
+  if (failed != 0.0) { p2p_release(c); return TBA_OK; }
   CUDA_OK(c, c->p2p_inbox_ptrs.alloc((size_t)W));
   CUDA_OK(c, c->p2p_flag_ptrs.alloc((size_t)W));
   CUDA_OK(c, cudaMemcpyAsync(c->p2p_inbox_ptrs.p, inbox.data(), (size_t)W * sizeof(double*), cudaMemcpyHostToDevice, c->stream));
@@ -437,33 +450,19 @@ P2pDev p2p_next(tba_context* c) {
   return d;
 }
 
-// One pass of the implicit Schur operator (MODE 0 matvec, 1 reduced rhs, 2 back-substitution) over every tile: the persistent
-// streaming kernel over the normal tiles, the tile-per-CTA kernel over the long tiles (tracks of 33..256 observations).
-template <int MODE>
-int launch_schur(tba_context* c, const double* xs, double* y, const int* done, const P2pDev& pp = P2pDev()) {
+// One pass of the implicit Schur operator (mode 0 matvec, 1 reduced rhs, 2 back-substitution) over every tile: the persistent
+// streaming kernel over the leading normal tiles, the tile-per-CTA kernel over the rest (the long tiles: tracks of 33..256
+// observations).
+int launch_schur(tba_context* c, int mode, const double* xs, double* y, const int* done, const P2pDev& pp = P2pDev()) {
   DevProblem& P = c->P;
-  int first_tile = 0;
-  if (c->stream_schur && c->exp_tred && c->n_normal_tiles > 0) {
-    const int n_slices = c->n_normal_tiles * (TILE / 32);
-#define F(M) { using Cfg = StreamCfg<M, MODE>; auto kfn = k_schur_stream<M, MODE>; \
-               const int grid = std::max(1, std::min(c->n_sm, (n_slices + Cfg::NW - 1) / Cfg::NW)); \
-               LAUNCH(c, kfn, grid, Cfg::NW * 32, Cfg::SMEM, P, xs, y, c->rep.p, done, n_slices, pp); }
-    DISPATCH_IMASK(c->imask, F)
-#undef F
-    first_tile = c->n_normal_tiles;
+  const KernelSet& k = c->ks;
+  if (k.n_stream_tiles > 0) {
+    const int n_slices = k.n_stream_tiles * (TILE / 32);
+    const auto& s = k.schur_stream[mode];
+    LAUNCH(c, s.fn, persistent_grid(c, s.nw, n_slices), s.nw * 32, s.smem, P, xs, y, c->rep.p, done, n_slices, pp);
   }
-  const int rest = P.n_tiles - first_tile;
-  if (rest > 0) {
-    if (c->exp_tred || MODE == 2) {
-#define F(M) { auto kfn = k_schur<M, MODE, true>; LAUNCH(c, kfn, rest, TILE, schur_smem(c), P, xs, y, c->rep.p, done, first_tile); }
-      DISPATCH_IMASK(c->imask, F)
-#undef F
-    } else {
-#define F(M) { auto kfn = k_schur<M, MODE, false>; LAUNCH(c, kfn, rest, TILE, schur_smem(c), P, xs, y, c->rep.p, done, first_tile); }
-      DISPATCH_IMASK(c->imask, F)
-#undef F
-    }
-  }
+  const int rest = P.n_tiles - k.n_stream_tiles;
+  if (rest > 0) LAUNCH(c, k.schur[mode], rest, TILE, k.schur_smem, P, xs, y, c->rep.p, done, k.n_stream_tiles);
   return TBA_OK;
 }
 
@@ -473,6 +472,7 @@ int launch_schur(tba_context* c, const double* xs, double* y, const int* done, c
 int stage_prepare(tba_context* c, double radius, bool* ok, bool defer_flag = false) {
   DevProblem& P = c->P;
   const tba_options& o = c->opt;
+  const KernelSet& k = c->ks;
   CUDA_OK(c, cudaMemsetAsync(c->flag.p, 0, sizeof(double), c->stream));
   LAUNCH(c, k_cs_diag, VB, VT, 0, P.ncs, lin_cn(c), c->sm.p, radius, o.min_lm_diagonal, o.max_lm_diagonal, c->D2.p);
   if (P.n_pt > 0) LAUNCH(c, k_point_blocks, (P.n_pt + 255) / 256, 256, 0, P, radius, o.min_lm_diagonal, o.max_lm_diagonal, c->flag.p);
@@ -487,48 +487,29 @@ int stage_prepare(tba_context* c, double radius, bool* ok, bool defer_flag = fal
   if (P.n_tiles > 0) {
     // normal tiles: ONE streaming pass over J for the reduced rhs and both families of SCHUR_JACOBI blocks (k_prepare_stream);
     // long tiles (and TBA_MATVEC=tile / IDENTITY preconditioner): the three tile kernels
-    int first_tile = 0;
-    if (c->stream_schur && c->exp_tred && precond && c->n_normal_tiles > 0) {
-      const int n_slices = c->n_normal_tiles * (TILE / 32);
+    const int first_tile = precond ? k.n_stream_tiles : 0;
+    if (first_tile > 0) {
+      const int n_slices = first_tile * (TILE / 32);
       const int pb = prof_begin(c);
-#define F(M) { using Cfg = PrepCfg<M>; auto kfn = k_prepare_stream<M>; \
-               const int grid = std::max(1, std::min(c->n_sm, (n_slices + Cfg::NW - 1) / Cfg::NW)); \
-               LAUNCH(c, kfn, grid, Cfg::NW * 32, Cfg::SMEM, P, yr, c->Sblk.p, c->Sblk.p + (size_t)P.n_cam * 21, c->rep.p, n_slices); }
-      DISPATCH_IMASK(c->imask, F)
-#undef F
+      LAUNCH(c, k.prepare_stream.fn, persistent_grid(c, k.prepare_stream.nw, n_slices), k.prepare_stream.nw * 32, k.prepare_stream.smem,
+             P, yr, c->Sblk.p, c->Sblk.p + (size_t)P.n_cam * 21, c->rep.p, n_slices);
       prof_end(c, 7, pb);
-      first_tile = c->n_normal_tiles;
     }
     const int rest = P.n_tiles - first_tile;
     if (rest > 0 && precond) {
       const int pb_ext = prof_begin(c);
-      if (c->exp_tred) {
-#define F(M) { auto kfn = k_precond_ext<M, true>; LAUNCH(c, kfn, rest, TILE, 0, P, c->Sblk.p, first_tile); }
-        DISPATCH_IMASK(c->imask, F)
-#undef F
-      } else {
-#define F(M) LAUNCH(c, k_precond_ext<M>, rest, TILE, 0, P, c->Sblk.p, first_tile)
-        DISPATCH_IMASK(c->imask, F)
-#undef F
-      }
+      LAUNCH(c, k.precond_ext, rest, TILE, 0, P, c->Sblk.p, first_tile);
       prof_end(c, 2, pb_ext);
       if (c->NI > 0) {
-        const size_t smem = (size_t)TILE * 4 * c->NI * sizeof(double) + 2 * TILE * sizeof(int);
         const int pb_intr = prof_begin(c);
-#define F(M) LAUNCH(c, k_precond_intr<M>, rest, TILE, smem, P, c->Sblk.p + (size_t)P.n_cam * 21, first_tile)
-        DISPATCH_IMASK(c->imask, F)
-#undef F
+        LAUNCH(c, k.precond_intr, rest, TILE, k.precond_intr_smem, P, c->Sblk.p + (size_t)P.n_cam * 21, first_tile);
         prof_end(c, 3, pb_intr);
       }
     }
     if (rest > 0) {
       const int pb_rhs = prof_begin(c);
-      if (first_tile == 0) { const int rc1 = launch_schur<1>(c, nullptr, yr, nullptr); if (rc1) return rc1; }
-      else {
-#define F(M) { auto kfn = k_schur<M, 1, true>; LAUNCH(c, kfn, rest, TILE, schur_smem(c), P, nullptr, yr, c->rep.p, nullptr, first_tile); }
-        DISPATCH_IMASK(c->imask, F)
-#undef F
-      }
+      if (first_tile == 0) { const int rc1 = launch_schur(c, 1, nullptr, yr, nullptr); if (rc1) return rc1; }
+      else LAUNCH(c, k.schur[1], rest, TILE, k.schur_smem, P, nullptr, yr, c->rep.p, nullptr, first_tile);
       prof_end(c, 4, pb_rhs);
     }
     if (P.single_group) LAUNCH(c, k_fold, 1, REPW, 0, c->rep.p, yr + P.ne, nullptr, nullptr);
@@ -566,7 +547,7 @@ int launch_matvec(tba_context* c, const int* done, bool defer_fold = false, cons
   DevProblem& P = c->P;
   if (P.n_tiles > 0) {
     const int pb = prof_begin(c);
-    const int rc = launch_schur<0>(c, c->xs.p, c->y.p, done, pp);
+    const int rc = launch_schur(c, 0, c->xs.p, c->y.p, done, pp);
     if (rc) return rc;
     prof_end(c, 0, pb);
     if (pp.world > 1) return TBA_OK;
@@ -687,13 +668,24 @@ int stage_backsub(tba_context* c) {
   CUDA_OK(c, cudaMemsetAsync(c->scal2.p, 0, 16 * sizeof(double), c->stream));
   if (P.n_tiles > 0) {
     const int pb_bs = prof_begin(c);
-    { const int rc2 = launch_schur<2>(c, c->xs.p, nullptr, nullptr); if (rc2) return rc2; }
+    { const int rc2 = launch_schur(c, 2, c->xs.p, nullptr, nullptr); if (rc2) return rc2; }
     prof_end(c, 5, pb_bs);
     LAUNCH(c, k_fold, 1, REPW, 0, c->rep.p, nullptr, nullptr, c->scal2.p);
   }
   // candidate = x + delta, step norm
   LAUNCH(c, k_candidate_cs, VB, VT, 0, P, c->xs.p, c->scal2.p, c->rank == 0 ? 1 : 0);
   if (P.n_pt > 0) LAUNCH(c, k_candidate_pt, small_grid(c, P.n_pt), 256, 0, P, c->scal2.p);
+  return TBA_OK;
+}
+
+// Cost at the candidate over every tile, added to scal2[0..2] = [cost, fixed, failed].  profile: record k_cost as span 6.
+int launch_candidate_cost(tba_context* c, bool profile) {
+  DevProblem& P = c->P;
+  if (P.n_tiles == 0) return TBA_OK;
+  const int pb = profile ? prof_begin(c) : -1;
+  LAUNCH(c, c->ks.cost, P.n_tiles, TILE, 0, P, P.ext_c, P.cam_s4_c, P.intr_c, P.pt_c, c->rep.p);
+  prof_end(c, 6, pb);
+  LAUNCH(c, k_fold, 1, REPW, 0, c->rep.p, nullptr, nullptr, c->scal2.p);
   return TBA_OK;
 }
 
@@ -705,20 +697,13 @@ int stage_evaluate_candidate(tba_context* c, double* cand_cost, double* mcc, dou
   // clock: its elapsed time rides in slot 8 of this all-reduce (the other ranks add 0), so every rank reads the same value.
   if (c->world > 1) LAUNCH(c, k_set_f64, 1, 1, 0, c->scal2.p + 8, c->rank == 0 ? elapsed_s : 0.0);
   LAUNCH(c, k_cam_prep, (P.n_cam + 127) / 128, 128, 0, P.n_cam, P.ext_c, P.cam_rec_c, P.cam_s4_c);
-  if (P.n_tiles > 0) {
-    const int pb_cost = prof_begin(c);
-    if (c->has_ext_models) { auto kfn = k_cost<true>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, P.ext_c, P.cam_s4_c, P.intr_c, P.pt_c, c->rep.p); }
-    else { auto kfn = k_cost<false>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, P.ext_c, P.cam_s4_c, P.intr_c, P.pt_c, c->rep.p); }
-    prof_end(c, 6, pb_cost);
-    LAUNCH(c, k_fold, 1, REPW, 0, c->rep.p, nullptr, nullptr, c->scal2.p);
-  }
+  int rc = launch_candidate_cost(c, true);
+  if (rc) return rc;
   // ||candidate|| over the non-constant blocks rides along (slots 6, 7): if the step is accepted it is the ||x|| the next
   // parameter-tolerance test needs -- no separate kernel + all-reduce + host round trip after the acceptance
   if (cand_xnorm) LAUNCH(c, k_xnorm, small_grid(c, std::max(P.n_pt, P.ne)), 256, 0, P, P.ext_c, P.intr_c, P.pt_c, c->blk_free.p, c->scal2.p, c->rank == 0 ? 1 : 0);
-  int rc = allreduce_sum(c, c->scal2.p, 9);
-  if (rc) return rc;
   double s[9];
-  rc = read_scal(c, c->scal2.p, 9, s);
+  rc = allreduce_read(c, c->scal2.p, 9, s);
   if (rc) return rc;
   *ok = s[2] == 0.0;
   *cand_cost = s[0];
@@ -733,10 +718,8 @@ int stage_xnorm(tba_context* c, double* xn) {
   DevProblem& P = c->P;
   CUDA_OK(c, cudaMemsetAsync(c->scal2.p, 0, 16 * sizeof(double), c->stream));
   LAUNCH(c, k_xnorm, small_grid(c, std::max(P.n_pt, P.ne)), 256, 0, P, P.ext, P.intr, P.pt, c->blk_free.p, c->scal2.p, c->rank == 0 ? 1 : 0);
-  int rc = allreduce_sum(c, c->scal2.p + 6, 2);
-  if (rc) return rc;
   double s[2];
-  rc = read_scal(c, c->scal2.p + 6, 2, s);
+  const int rc = allreduce_read(c, c->scal2.p + 6, 2, s);
   if (rc) return rc;
   *xn = std::sqrt(s[0] + s[1]);
   return TBA_OK;
@@ -803,13 +786,7 @@ int run_block_stage(tba_context* c) {
     CUDA_OK(c, cudaMemcpyAsync(c->d_blk_active.p, active.data(), (size_t)nb, cudaMemcpyHostToDevice, c->stream));
     CUDA_OK(c, cudaMemsetAsync(c->d_blk_acc.p, 0, acc.size() * 8, c->stream));
     if (KIND == kBlockCamera) LAUNCH(c, k_cam_prep, (nb + 127) / 128, 128, 0, nb, c->d_blk_vals.p, c->d_blk_rec.p, (double*)nullptr);
-    if (P.n_tiles > 0 && pass == 0) {
-      auto kfn = c->has_ext_models ? k_block_pass<KIND, true, false> : k_block_pass<KIND, false, false>;
-      LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, A);
-    } else if (P.n_tiles > 0) {
-      auto kfn = c->has_ext_models ? k_block_pass<KIND, true, true> : k_block_pass<KIND, false, true>;
-      LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, A);
-    }
+    if (P.n_tiles > 0) LAUNCH(c, c->ks.block_pass[KIND][pass != 0], P.n_tiles, TILE, 0, P, A);
     const int rc = allreduce_sum(c, c->d_blk_acc.p, acc.size());
     if (rc) return rc;
     CUDA_OK(c, cudaMemcpyAsync(acc.data(), c->d_blk_acc.p, acc.size() * 8, cudaMemcpyDeviceToHost, c->stream));
@@ -849,20 +826,14 @@ int stage_inner_iterations(tba_context* c, double* inner_cost, bool* ok) {
     CUDA_OK(c, c->d_inner_status.alloc((size_t)P.n_pt));  // no-ops: sized at upload
     CUDA_OK(c, c->d_inner_cost2.alloc((size_t)P.n_pt * 2));
     const DevProblem Q = candidate_view(P);
-    auto kfn = c->has_ext_models ? k_adjust_tracks<true> : k_adjust_tracks<false>;
-    LAUNCH(c, kfn, (P.n_pt + 63) / 64, 64, 0, Q, c->pt_slot.p, c->pt_len.p, po, c->d_inner_status.p, c->d_inner_cost2.p);
+    LAUNCH(c, c->ks.adjust_tracks, (P.n_pt + 63) / 64, 64, 0, Q, c->pt_slot.p, c->pt_len.p, po, c->d_inner_status.p, c->d_inner_cost2.p);
   }
   // cost at the refined candidate
   CUDA_OK(c, cudaMemsetAsync(c->scal2.p, 0, 3 * sizeof(double), c->stream));
-  if (P.n_tiles > 0) {
-    if (c->has_ext_models) { auto kfn = k_cost<true>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, P.ext_c, P.cam_s4_c, P.intr_c, P.pt_c, c->rep.p); }
-    else { auto kfn = k_cost<false>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, P.ext_c, P.cam_s4_c, P.intr_c, P.pt_c, c->rep.p); }
-    LAUNCH(c, k_fold, 1, REPW, 0, c->rep.p, nullptr, nullptr, c->scal2.p);
-  }
-  rc = allreduce_sum(c, c->scal2.p, 3);
+  rc = launch_candidate_cost(c, false);
   if (rc) return rc;
   double s3[3];
-  rc = read_scal(c, c->scal2.p, 3, s3);
+  rc = allreduce_read(c, c->scal2.p, 3, s3);
   if (rc) return rc;
   *inner_cost = s3[0];
   *ok = s3[2] == 0.0;
@@ -874,10 +845,8 @@ int stage_step_norm(tba_context* c, double* step_norm) {
   DevProblem& P = c->P;
   CUDA_OK(c, cudaMemsetAsync(c->scal2.p + 4, 0, 2 * sizeof(double), c->stream));
   LAUNCH(c, k_xdiff, 256, 256, 0, P, c->blk_free.p, c->scal2.p, c->rank == 0 ? 1 : 0);
-  int rc = allreduce_sum(c, c->scal2.p + 4, 2);
-  if (rc) return rc;
   double s2[2];
-  rc = read_scal(c, c->scal2.p + 4, 2, s2);
+  const int rc = allreduce_read(c, c->scal2.p + 4, 2, s2);
   if (rc) return rc;
   *step_norm = std::sqrt(s2[0] + s2[1]);
   return TBA_OK;
@@ -897,6 +866,61 @@ int check_options(tba_context* c, const tba_options* o) {
   }
   if (o->linear_solver_type == TBA_ITERATIVE_SCHUR && o->preconditioner_type != TBA_PRECOND_SCHUR_JACOBI && o->preconditioner_type != TBA_PRECOND_IDENTITY) { set_err(c, "preconditioner_type %d unsupported (SCHUR_JACOBI or IDENTITY)", o->preconditioner_type); return TBA_ERR_UNSUPPORTED; }
   if (o->loss_function_type < 0 || o->loss_function_type > 5) { set_err(c, "invalid loss function type %d", o->loss_function_type); return TBA_ERR_INVALID_ARGUMENT; }
+  return TBA_OK;
+}
+
+// The kernels that depend on the intrinsics column set M.
+template <uint32_t M>
+void select_mask_kernels(const tba_context* c, KernelSet& k) {
+  const bool tred = c->exp_tred;
+  if (c->exp_lin_occ) k.linearize = tred ? k_linearize<M, false, true, 3> : k_linearize<M, false, false, 3>;
+  else k.linearize = tred ? k_linearize<M, false, true> : k_linearize<M>;
+  k.schur[0] = tred ? k_schur<M, 0, true> : k_schur<M, 0, false>;
+  k.schur[1] = tred ? k_schur<M, 1, true> : k_schur<M, 1, false>;
+  k.schur[2] = k_schur<M, 2, true>;  // back-substitution runs the TRED variant under either TBA_TRED setting
+  k.schur_smem = (size_t)(14 + 2 * popcount10(M) + 2) * TILE * sizeof(double);
+  k.schur_stream[0] = {k_schur_stream<M, 0>, StreamCfg<M, 0>::NW, StreamCfg<M, 0>::SMEM};
+  k.schur_stream[1] = {k_schur_stream<M, 1>, StreamCfg<M, 1>::NW, StreamCfg<M, 1>::SMEM};
+  k.schur_stream[2] = {k_schur_stream<M, 2>, StreamCfg<M, 2>::NW, StreamCfg<M, 2>::SMEM};
+  k.prepare_stream = {k_prepare_stream<M>, PrepCfg<M>::NW, PrepCfg<M>::SMEM};
+  k.precond_ext = tred ? k_precond_ext<M, true> : k_precond_ext<M>;
+  k.precond_intr = k_precond_intr<M>;
+  k.precond_intr_smem = (size_t)TILE * 4 * popcount10(M) * sizeof(double) + 2 * TILE * sizeof(int);
+}
+
+// Fills c->ks for an upload whose intrinsics column set is `imask` and opts its kernels in to the shared memory they launch with.
+// The streaming kernels take the leading n_normal_tiles tiles unless TBA_MATVEC=tile or TBA_TRED=0 switched them off.
+int select_kernels(tba_context* c, uint32_t imask, int n_normal_tiles) {
+  KernelSet& k = c->ks;
+  k = KernelSet();
+  switch (imask) {  // the sets of kMasks
+    case 0x000u: select_mask_kernels<0x000u>(c, k); break;
+    case 0x001u: select_mask_kernels<0x001u>(c, k); break;
+    case 0x061u: select_mask_kernels<0x061u>(c, k); break;
+    case 0x0E1u: select_mask_kernels<0x0E1u>(c, k); break;
+    case 0x07Fu: select_mask_kernels<0x07Fu>(c, k); break;
+    default: select_mask_kernels<0x3FFu>(c, k); break;
+  }
+  // FISHEYE / FOV / DIVISION_UNDISTORTION (imask 0x3FF): the dual-number instantiations.  nvcc emits kernel templates in the order
+  // of their first reference, and the code generated for the dual-number kernels that share device functions depends on that
+  // order: keep k_linearize<0x3FF, true> the first kernel template this file names.
+  const bool ext = c->has_ext_models;
+  if (ext) k.linearize = k_linearize<0x3FFu, true>;
+  k.cost = ext ? k_cost<true> : k_cost<false>;
+  k.adjust_tracks = ext ? k_adjust_tracks<true> : k_adjust_tracks<false>;
+  k.filter_tracks = ext ? k_filter_tracks<true> : k_filter_tracks<false>;
+  k.estimate_tracks = ext ? k_estimate_tracks<true> : k_estimate_tracks<false>;
+  k.block_pass[kBlockCamera][0] = ext ? k_block_pass<kBlockCamera, true, false> : k_block_pass<kBlockCamera, false, false>;
+  k.block_pass[kBlockCamera][1] = ext ? k_block_pass<kBlockCamera, true, true> : k_block_pass<kBlockCamera, false, true>;
+  k.block_pass[kBlockGroup][0] = ext ? k_block_pass<kBlockGroup, true, false> : k_block_pass<kBlockGroup, false, false>;
+  k.block_pass[kBlockGroup][1] = ext ? k_block_pass<kBlockGroup, true, true> : k_block_pass<kBlockGroup, false, true>;
+  k.n_stream_tiles = c->stream_schur && c->exp_tred ? n_normal_tiles : 0;
+  if (c->NI > 0) CUDA_OK(c, cudaFuncSetAttribute(k.precond_intr, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.precond_intr_smem));
+  for (int mode = 0; mode < 3; ++mode) {
+    CUDA_OK(c, cudaFuncSetAttribute(k.schur[mode], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.schur_smem));
+    CUDA_OK(c, cudaFuncSetAttribute(k.schur_stream[mode].fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.schur_stream[mode].smem));
+  }
+  CUDA_OK(c, cudaFuncSetAttribute(k.prepare_stream.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.prepare_stream.smem));
   return TBA_OK;
 }
 
@@ -1083,15 +1107,7 @@ int tba_upload(tba_context* c, const tba_options* options, const tba_problem* p)
     tmp.insert(tmp.end(), cnt_g.begin(), cnt_g.end());
     tmp.push_back((double)c->n_free_pt);
     tmp.push_back(local_err != TBA_OK ? 1.0 : 0.0);  // number of ranks whose shard failed validation
-    rc = [&]() -> int {
-      CUDA_OK(c, c->scal2.alloc(std::max<size_t>(tmp.size(), 16)));
-      CUDA_OK(c, cudaMemcpyAsync(c->scal2.p, tmp.data(), tmp.size() * 8, cudaMemcpyHostToDevice, c->stream));
-      int r2 = allreduce_sum(c, c->scal2.p, tmp.size());
-      if (r2) return r2;
-      CUDA_OK(c, cudaMemcpyAsync(tmp.data(), c->scal2.p, tmp.size() * 8, cudaMemcpyDeviceToHost, c->stream));
-      CUDA_OK(c, cudaStreamSynchronize(c->stream));
-      return TBA_OK;
-    }();
+    rc = allreduce_host(c, tmp.data(), tmp.size());
     if (rc) return rc;
     if (tmp.back() != 0.0) {  // some rank failed: every rank returns an error, nobody is left inside a collective
       if (local_err == TBA_OK) { set_err(c, "upload failed on %d other rank(s) (invalid observation indices or over-long track in their shard)", (int)tmp.back()); return TBA_ERR_INVALID_ARGUMENT; }
@@ -1110,10 +1126,8 @@ int tba_upload(tba_context* c, const tba_options* options, const tba_problem* p)
   std::vector<int>& tile_nruns = H.tile_nruns;
   std::vector<uint8_t>& tile_flags = H.tile_flags;
   c->n_free_cs = H.n_free_cs;
-  c->imask = 0x3FFu;
-  for (uint32_t m : kMasks) if ((H.union_free & ~m) == 0) { c->imask = m; break; }
-  if (c->has_ext_models) c->imask = 0x3FFu;  // one instantiation for the other models: every intrinsics column stored
-  c->NI = popcount10(c->imask);
+  const uint32_t imask = c->has_ext_models ? 0x3FFu : intrinsics_mask(H.union_free);  // other models: every intrinsics column stored
+  c->NI = popcount10(imask);
   c->NJ = 14 + 2 * c->NI;
   const int npk = (int)H.pk2caller.size();
   const int n_long = H.n_long;
@@ -1227,44 +1241,21 @@ int tba_upload(tba_context* c, const tba_options* options, const tba_problem* p)
   P.tile_pt_begin = c->tile_pt_begin.p; P.tile_nruns = c->tile_nruns.p; P.tile_flags = c->tile_flags.p; P.xy = c->xy.p; P.J = c->J.p; P.res = c->res.p;
   P.Hpp = c->Hpp.p; P.gp = c->gp.p; P.Mp = c->Mp.p; P.sp = c->sp.p; P.dpt = c->dpt.p; P.pt_const = c->pt_const.p;
   { const char* e = getenv("TBA_ABLATE"); P.ablate = e ? atoi(e) : 0; }  // timing diagnostics only (wrong results): see k_schur
-  if (c->NI > 0) {
-    const int smem = TILE * 4 * c->NI * (int)sizeof(double) + 2 * TILE * (int)sizeof(int);
-#define F(M) CUDA_OK(c, cudaFuncSetAttribute(k_precond_intr<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem))
-    DISPATCH_IMASK(c->imask, F)
-#undef F
-  }
-  {
-    const int smem = (int)schur_smem(c);
-#define F(M)                                                                                                        \
-  CUDA_OK(c, cudaFuncSetAttribute(k_schur<M, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));        \
-  CUDA_OK(c, cudaFuncSetAttribute(k_schur<M, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));       \
-  CUDA_OK(c, cudaFuncSetAttribute(k_schur<M, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));        \
-  CUDA_OK(c, cudaFuncSetAttribute(k_schur<M, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));       \
-  CUDA_OK(c, cudaFuncSetAttribute(k_schur<M, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));        \
-  CUDA_OK(c, cudaFuncSetAttribute(k_schur_stream<M, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)StreamCfg<M, 0>::SMEM)); \
-  CUDA_OK(c, cudaFuncSetAttribute(k_schur_stream<M, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)StreamCfg<M, 1>::SMEM)); \
-  CUDA_OK(c, cudaFuncSetAttribute(k_schur_stream<M, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)StreamCfg<M, 2>::SMEM)); \
-  CUDA_OK(c, cudaFuncSetAttribute(k_prepare_stream<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PrepCfg<M>::SMEM));
-    DISPATCH_IMASK(c->imask, F)
-#undef F
-  }
-  c->n_normal_tiles = 0;
-  for (int t = 0; t < n_tiles; ++t) c->n_normal_tiles += (tile_flags[t] & 1) ? 0 : 1;
+  int n_normal_tiles = 0;  // tiles whose tracks fit a warp slice (they precede the long tiles)
+  for (int t = 0; t < n_tiles; ++t) n_normal_tiles += (tile_flags[t] & 1) ? 0 : 1;
+  rc = select_kernels(c, imask, n_normal_tiles);
+  if (rc) return rc;
   {
     // multi-GPU: peer-memory inbox for the fused matvec + all-reduce; used only if EVERY rank runs its whole shard through the
     // streaming kernel (a rank with long tiles or without tiles would not push) -- agreed on collectively, here
-    const int rcp = p2p_setup(c, ncs);
-    if (rcp) return rcp;
+    rc = p2p_setup(c, ncs);
+    if (rc) return rc;
     c->p2p_use = false;
     if (c->world > 1 && c->p2p_ok) {
-      const double mine = (c->stream_schur && c->exp_tred && c->n_normal_tiles > 0 && c->n_normal_tiles == n_tiles) ? 0.0 : 1.0;
-      double others = 0.0;
-      CUDA_OK(c, cudaMemcpyAsync(c->scal2.p, &mine, 8, cudaMemcpyHostToDevice, c->stream));
-      const int r2 = allreduce_sum(c, c->scal2.p, 1);
-      if (r2) return r2;
-      CUDA_OK(c, cudaMemcpyAsync(&others, c->scal2.p, 8, cudaMemcpyDeviceToHost, c->stream));
-      CUDA_OK(c, cudaStreamSynchronize(c->stream));
-      c->p2p_use = others == 0.0;
+      double n_pushless = (c->ks.n_stream_tiles > 0 && c->ks.n_stream_tiles == n_tiles) ? 0.0 : 1.0;  // ranks that would not push
+      rc = allreduce_host(c, &n_pushless, 1);
+      if (rc) return rc;
+      c->p2p_use = n_pushless == 0.0;
     }
   }
   c->have_scale = false;
@@ -1532,14 +1523,10 @@ int tba_set_profiling(tba_context* c, int enable) {
 // out[4] = observation slots, out[5] = valid observations, out[6] = packed points, out[7] = doubles stored per observation
 int tba_get_profile(tba_context* c, double* out) {
   if (!c || !out) return TBA_ERR_INVALID_ARGUMENT;
-  CUDA_OK(c, cudaSetDevice(c->device));
-  CUDA_OK(c, cudaStreamSynchronize(c->stream));
-  for (int w = 0; w < 2; ++w) {
-    double tot = 0;
-    for (auto& sp : c->ev_spans[w]) { float ms = 0; cudaEventElapsedTime(&ms, c->ev_pool[sp.first], c->ev_pool[sp.second]); tot += ms; }
-    out[2 * w] = tot; out[2 * w + 1] = (double)c->ev_spans[w].size();
-  }
-  out[1] = (double)c->real_matvecs;  // early-exited launches (after convergence inside a batch) cost ~2 us and do no work
+  double stages[16];
+  const int rc = tba_get_profile_stages(c, stages);
+  if (rc) return rc;
+  std::copy(stages, stages + 4, out);
   out[4] = (double)c->n_slots; out[5] = (double)c->n_obs; out[6] = (double)c->n_pt; out[7] = (double)c->NJ;
   return TBA_OK;
 }
@@ -1556,7 +1543,7 @@ int tba_get_profile_stages(tba_context* c, double* out) {
     for (auto& sp : c->ev_spans[w]) { float ms = 0; cudaEventElapsedTime(&ms, c->ev_pool[sp.first], c->ev_pool[sp.second]); tot += ms; }
     out[2 * w] = tot; out[2 * w + 1] = (double)c->ev_spans[w].size();
   }
-  out[1] = (double)c->real_matvecs;
+  out[1] = (double)c->real_matvecs;  // early-exited launches (after convergence inside a batch) cost ~2 us and do no work
   return TBA_OK;
 }
 
@@ -1578,8 +1565,7 @@ int tba_filter_tracks(tba_context* c, double max_inlier_reprojection_error, doub
   // the per-camera rotation records must describe the CURRENT extrinsics
   LAUNCH(c, k_cam_prep, (P.n_cam + 127) / 128, 128, 0, P.n_cam, P.ext, P.cam_rec, P.cam_s4);
   if (P.n_pt > 0) {
-    auto kfn = c->has_ext_models ? k_filter_tracks<true> : k_filter_tracks<false>;
-    LAUNCH(c, kfn, (P.n_pt + 127) / 128, 128, 0, P, c->pt_slot.p, c->pt_len.p, max_sq, cos_min, d_status.p, c->pt_stat.p);
+    LAUNCH(c, c->ks.filter_tracks, (P.n_pt + 127) / 128, 128, 0, P, c->pt_slot.p, c->pt_len.p, max_sq, cos_min, d_status.p, c->pt_stat.p);
   }
   std::vector<uint8_t> hs((size_t)P.n_pt);
   std::vector<double> hm((size_t)P.n_pt);
@@ -1646,8 +1632,7 @@ int tba_adjust_tracks(tba_context* c, const tba_options* options, uint8_t* statu
   CUDA_OK(c, d_cost2.alloc((size_t)P.n_pt * 2));
   LAUNCH(c, k_cam_prep, (P.n_cam + 127) / 128, 128, 0, P.n_cam, P.ext, P.cam_rec, P.cam_s4);
   if (P.n_pt > 0) {
-    auto kfn = c->has_ext_models ? k_adjust_tracks<true> : k_adjust_tracks<false>;
-    LAUNCH(c, kfn, (P.n_pt + 63) / 64, 64, 0, P, c->pt_slot.p, c->pt_len.p, point_lm_options(*options), d_status.p, d_cost2.p);
+    LAUNCH(c, c->ks.adjust_tracks, (P.n_pt + 63) / 64, 64, 0, P, c->pt_slot.p, c->pt_len.p, point_lm_options(*options), d_status.p, d_cost2.p);
   }
   const int rc = gather_track_outputs(c, d_status.p, d_cost2.p, kTrackSkipped, status, initial_cost, final_cost);
   if (rc) return rc;
@@ -1676,8 +1661,7 @@ int tba_estimate_tracks(tba_context* c, const tba_options* ba_options, double ma
   double* ray = P.J;
   if (c->n_slots > 0) LAUNCH(c, k_track_rays, (unsigned)((c->n_slots + 255) / 256), 256, 0, P, (long long)c->n_slots, ray);
   if (P.n_pt > 0) {
-    auto kfn = c->has_ext_models ? k_estimate_tracks<true> : k_estimate_tracks<false>;
-    LAUNCH(c, kfn, (P.n_pt + 63) / 64, 64, 0, P, c->pt_slot.p, c->pt_len.p, ray, o, d_status.p, d_cost2.p);
+    LAUNCH(c, c->ks.estimate_tracks, (P.n_pt + 63) / 64, 64, 0, P, c->pt_slot.p, c->pt_len.p, ray, o, d_status.p, d_cost2.p);
   }
   // caller points without any observation: "view_ids.size() < 2" -> bad angle bucket
   const int rc = gather_track_outputs(c, d_status.p, d_cost2.p, kTrackBadAngle, status, nullptr, nullptr);
@@ -1938,8 +1922,7 @@ int tba_debug_pack(const tba_problem* p, int64_t cap_slots, int64_t* sizes_out, 
   std::vector<double> cnt_c(p->n_cam, 0.0), cnt_g(p->n_group, 0.0);
   for (int i = 0; i < p->n_cam; ++i) { cnt_c[i] = H.cnt_cam[i]; cnt_g[p->cam_group[i]] += H.cnt_cam[i]; }
   pack_masks_and_tiles(p, cnt_c, cnt_g, &H);
-  uint32_t imask = 0x3FFu;
-  for (uint32_t m : kMasks) if ((H.union_free & ~m) == 0) { imask = m; break; }
+  const uint32_t imask = intrinsics_mask(H.union_free);
   sizes_out[0] = H.n_tiles; sizes_out[1] = H.n_slots; sizes_out[2] = (int64_t)H.pk2caller.size(); sizes_out[3] = H.n_long;
   sizes_out[4] = popcount10(imask); sizes_out[5] = imask;
   if (H.n_slots > cap_slots) return TBA_ERR_INVALID_ARGUMENT;
@@ -2022,15 +2005,10 @@ int tba_debug_evaluate_step(tba_context* c, double* candidate_cost) {
   DevProblem& P = c->P;
   CUDA_OK(c, cudaMemsetAsync(c->scal2.p, 0, 3 * sizeof(double), c->stream));
   LAUNCH(c, k_cam_prep, (P.n_cam + 127) / 128, 128, 0, P.n_cam, P.ext_c, P.cam_rec_c, P.cam_s4_c);
-  if (P.n_tiles > 0) {
-    if (c->has_ext_models) { auto kfn = k_cost<true>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, P.ext_c, P.cam_s4_c, P.intr_c, P.pt_c, c->rep.p); }
-    else { auto kfn = k_cost<false>; LAUNCH(c, kfn, P.n_tiles, TILE, 0, P, P.ext_c, P.cam_s4_c, P.intr_c, P.pt_c, c->rep.p); }
-    LAUNCH(c, k_fold, 1, REPW, 0, c->rep.p, nullptr, nullptr, c->scal2.p);
-  }
-  int rc = allreduce_sum(c, c->scal2.p, 3);
+  int rc = launch_candidate_cost(c, false);
   if (rc) return rc;
   double s[3];
-  rc = read_scal(c, c->scal2.p, 3, s);
+  rc = allreduce_read(c, c->scal2.p, 3, s);
   if (rc) return rc;
   if (candidate_cost) *candidate_cost = s[0] + s[1];
   return s[2] == 0.0 ? TBA_OK : TBA_ERR_INVALID_ARGUMENT;

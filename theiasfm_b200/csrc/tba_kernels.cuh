@@ -94,7 +94,7 @@ __device__ __forceinline__ double seg_reduce(double v, int key, int lane) {
 
 // The same reduction when the run structure is known from a ballot of the run heads: lane + o belongs to lane's run iff
 // lane + o <= run_last (runs are contiguous), so the key does not have to be shuffled along with every value -- 5 shuffles per
-// reduced value instead of 10 (experiment switch TBA_FAST_SEG=1; bit-identical sums: same additions in the same order).
+// reduced value instead of 10 (bit-identical sums: same additions in the same order).
 __device__ __forceinline__ double seg_reduce_to(double v, int run_last, int lane) {
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) {
@@ -115,7 +115,7 @@ __device__ __forceinline__ void red_add(double* p, double v) {
 #endif
 }
 
-// Experiment TBA_TRED=1 ("transposed" RED emission).  A lane-per-observation RED of an N-double camera row touches 32
+// Transposed RED emission (default; TBA_TRED=0: lane-per-row REDs).  A lane-per-observation RED of an N-double camera row touches 32
 // different 32-byte sectors per instruction (32 cameras), i.e. N x 32 sector operations at the L2 atomic units, which
 // is what bounds these kernels (profiles/: k_precond_ext 88 % lts throughput at one sector operation per RED).  Here
 // the warp first stages its 32 rows in shared memory ([32][N] doubles, lane-major) and then emits them element-major:
@@ -284,7 +284,7 @@ __global__ void __launch_bounds__(TILE, MINB) k_linearize(DevProblem P, double* 
   }
   // camera-side gradient and squared column norms: J_c = [-h Ja | Jw]
   if (TRED && !long_tile) {
-    // experimental (TBA_TRED=1): both 6-rows staged per warp in the (idle on normal tiles) s_acc area, emitted element-major
+    // transposed RED emission: both 6-rows staged per warp in the (idle on normal tiles) s_acc area, emitted element-major
     double gv[6], cv[6];
 #pragma unroll
     for (int j = 0; j < 3; ++j) {
@@ -600,15 +600,13 @@ __device__ __forceinline__ void sym4_mul(const double* __restrict__ M, const dou
 // ---------------------------------------------------- TMA (bulk async copy) helpers
 #ifdef TBA_EMULATE
 // CPU emulation build (tests/emu/cuda_emu.h): the bulk copy is a memcpy by the issuing lane, the mbarrier a flag the other lanes
-// poll (yielding to the fiber scheduler), the bulk reduction an in-place add.
+// poll (yielding to the fiber scheduler).
 // *bar counts the completed phases: the issuing lane's sequence "expect_tx, bulk copy, bulk copy ..." runs without a yield in
 // between, so a phase is complete as soon as its expect_tx is visible; wait(parity) passes once phase `parity` is over.
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t) { *bar = 0; }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t) { *bar += 1; }
 __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t*) { memcpy(dst, src, bytes); }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) { while ((*bar & 1u) == parity) emu_yield(); }
-__device__ __forceinline__ void bulk_red_add_f64(double* dst, const double* src_smem, uint32_t bytes) { for (uint32_t i = 0; i < bytes / 8; ++i) dst[i] += src_smem[i]; }
-__device__ __forceinline__ void bulk_commit_and_wait_read() {}
 __device__ __forceinline__ void fence_proxy_async_smem() {}
 #else
 // cp.async.bulk global -> shared::cta completing on an mbarrier (SASS: UBLKCP + SYNCS.ARRIVE.TRANS64).
@@ -639,18 +637,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
 // Never a silent hang: a bulk copy that does not land within ~2 s (4e9 SM cycles) is a bug -- report it and abort the kernel
 // (the launch then fails with a CUDA error that the engine returns to the caller).
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-#ifdef TBA_MBAR_SIMPLE
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-  return;
-#endif
   if (mbar_try_wait(bar, parity)) return;
   const long long t0 = clock64();
   while (!mbar_try_wait(bar, parity)) {
@@ -661,17 +647,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
-// Bulk reduction shared -> global (TMA): dst[0..bytes) += src[0..bytes) element-wise in fp64, asynchronously.
-// bytes multiple of 16, both addresses 16-byte aligned.  Experimental path (TBA_MATVEC_BULKRED=1): replaces the six
-// per-observation RED.ADD.F64 of the matvec by ONE 48-byte bulk reduction issued from a staged shared-memory row.
-__device__ __forceinline__ void bulk_red_add_f64(double* dst, const double* src_smem, uint32_t bytes) {
-  asm volatile("cp.reduce.async.bulk.global.shared::cta.bulk_group.add.f64 [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(src_smem)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit_and_wait_read() {
-  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-  asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-}
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 #endif  // TBA_EMULATE
@@ -1105,24 +1080,11 @@ k_schur_stream(DevProblem P, const double* __restrict__ xs, double* __restrict__
 #define JH(j) Jt[(12 + (j)) * 32]
 #define JI(j) Jt[(14 + (j)) * 32]
     double w0 = 0.0, w1 = 0.0, r0 = 0.0, r1 = 0.0;
-    // the whole row set of this lane in registers: every element of J is read from shared memory exactly once
-    double ja[6], jh[2], jw[6], ji[2 * NI + 1];
+    // the point rows of this lane in registers (each is used by both products); the camera rows are read where they are used
+    double ja[6], jh[2];
 #pragma unroll
     for (int j = 0; j < 6; ++j) ja[j] = JA(j);
     jh[0] = JH(0); jh[1] = JH(1);
-#ifndef TBA_STREAM_CACHE_J
-#define TBA_STREAM_CACHE_J 0
-#endif
-    if (TBA_STREAM_CACHE_J && MODE != 2) {
-#pragma unroll
-      for (int j = 0; j < 6; ++j) jw[j] = JW(j);
-#pragma unroll
-      for (int j = 0; j < 2 * NI; ++j) ji[j] = JI(j);
-    }
-#undef JW
-#undef JI
-#define JW(j) ((TBA_STREAM_CACHE_J && MODE != 2) ? jw[j] : Jt[(6 + (j)) * 32])
-#define JI(j) ((TBA_STREAM_CACHE_J && MODE != 2) ? ji[j] : Jt[(14 + (j)) * 32])
     if (valid) {
       if (MODE != 0) { r0 = sR[lane]; r1 = sR[32 + lane]; }
       if (MODE != 1) {
@@ -1538,7 +1500,7 @@ __global__ void __launch_bounds__(TILE) k_precond_ext(DevProblem P, double* __re
   const size_t slot = (size_t)tile * TILE + tid;
   const int cam = P.slot_cam[slot];
   if (TRED) {
-    // experimental (TBA_TRED=1): the 21 block entries of every observation staged per warp, emitted element-major
+    // transposed RED emission: the 21 block entries of every observation staged per warp, emitted element-major
     __shared__ double s_stage[TILE / 32][32 * 21];
     __shared__ int s_base[TILE / 32][32];
     double v[21];
